@@ -315,9 +315,11 @@ def run_reference(opt):
     t0 = time.perf_counter()
     tv_sum = 0.0
     for k in range(opt.steps):
-        _, tv, _ = ref.frame(scenes[k % 2])
+        out, tv, _ = ref.frame(scenes[k % 2])
         tv_sum += tv
     dt = time.perf_counter() - t0
+    if opt.dump_outputs:
+        write_outputs(host_outputs(out), opt.dump_outputs)
     fps = opt.steps / dt
     cfg = workload_config(wl, 1, "cpu")
     cfg["precision"] = "fp32 (PyTorch CPU)"
@@ -338,6 +340,35 @@ def run_reference(opt):
 # GPU arm
 # ------------------------------------------------------------------------------------------------------------------
 HEADS = ("cls_preds", "reg_preds", "dir_preds")
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def host_outputs(out):
+    """Host copies of every tensor in a frame's output dict (list entries as <key>_<i>): float32, or float64 for float64 and
+    integer tensors."""
+    import torch
+    arrays = {}
+    for k, v in out.items():
+        for name, t in ([(f"{k}_{i}", t) for i, t in enumerate(v)] if isinstance(v, (list, tuple)) else [(k, v)]):
+            if torch.is_tensor(t):
+                wide = t.dtype == torch.float64 or not t.is_floating_point()
+                arrays[name] = t.detach().to("cpu", torch.float64 if wide else torch.float32).numpy()
+    return arrays
+
+
+def write_outputs(arrays, directory):
+    """DIR/<name>.npy per array.  Above DUMP_LIMIT_BYTES in all, every array is replaced by the same fraction of its elements
+    (flattened, at positions drawn from a generator seeded by the array's name), so the files stay comparable between runs."""
+    import zlib
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = DUMP_LIMIT_BYTES / total
+        for name, a in arrays.items():
+            idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).choice(a.size, int(a.size * keep), replace=False))
+            arrays[name] = a.reshape(-1)[idx]
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def parity_record(gpu_out, ref_out, precision, what):
@@ -572,9 +603,14 @@ def main():
     ap.add_argument("--inflight", type=int, default=2, help="captured frames in flight for `value` (N graphs on N streams, heal_b200.graph.FrameInterleaver); 1 = strictly one frame after the other (the number reported as `latency`)")
     ap.add_argument("--pipeline-depth", type=int, default=2, help="e2e: captured frames in flight in FramePipeline (results are delivered depth-1 submits later)")
     ap.add_argument("--no-pipeline", action="store_true", help="e2e: one stream, H2D -> frame -> D2H back to back (no copy/compute overlap)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed frame as DIR/<name>.npy (float32; float64 where "
+                         "the output is float64 or integer); the inputs are seeded, so two builds can be compared output for output")
     opt = ap.parse_args()
     ref = opt.impl == "reference"
     opt.steps = opt.steps if opt.steps is not None else (5 if ref else 20)
+    if opt.steps < 1:
+        ap.error("--steps must be at least 1")
     opt.warmup = opt.warmup if opt.warmup is not None else (1 if ref else 3)
     opt.warmup = max(opt.warmup, 3) if not ref else opt.warmup
     if opt.precision is None:
@@ -676,9 +712,14 @@ def run_gpu(opt):
         if rank == 0:
             sampler.start()
         # ---- timed region: K frames, ONE device-event interval, inputs resident in HBM ----
+        last = {}
+
+        def frame_timed(i):
+            last["out"] = frame_dev(i)
         l0 = lib.heal_launch_count()
-        serial_ms = time_frames(frame_dev, opt.steps, barrier)
+        serial_ms = time_frames(frame_timed, opt.steps, barrier)
         total_ms = serial_ms
+        dumped = host_outputs(last["out"]) if opt.dump_outputs and rank == 0 else None    # graph buffers are replayed again below
         inflight = 1
         if fg is not None and opt.inflight > 1:
             # `value`: N captured frames in flight on N streams (frame i+1's latency-bound head runs in the gaps of frame i); the
@@ -688,7 +729,7 @@ def run_gpu(opt):
 
             def frame_il(i):
                 t = wl.devin[i % len(wl.devin)]
-                il.submit(t["points"], t["offsets"], t["pairwise"])
+                return il.submit(t["points"], t["offsets"], t["pairwise"])
             for w in range(max(opt.warmup, 2 * opt.inflight)):
                 frame_il(w)
             il.join(begin=False)
@@ -697,11 +738,13 @@ def run_gpu(opt):
             e0.record()
             il.join(begin=True)
             for k in range(opt.steps):
-                frame_il(k)
+                last["out"] = frame_il(k)
             il.join(begin=False)
             e1.record()
             barrier()
             total_ms = e0.elapsed_time(e1)
+            if dumped is not None:
+                dumped = host_outputs(last["out"])             # `value` comes from this loop: its last frame is the one to show
             inflight = opt.inflight
             del il
             torch.cuda.empty_cache()
@@ -867,7 +910,7 @@ def run_gpu(opt):
             torch.cuda.empty_cache()
             for name in ("c1", "c3", "c4"):
                 try:
-                    secondary[name] = run_secondary_workload(name, "bf16" if name == "c4" else opt.precision, dev, peaks)
+                    secondary[name] = run_secondary_workload(name, "bf16" if name == "c4" else opt.precision, dev, peaks, opt.steps)
                 except Exception as e:
                     import traceback
                     sys.stderr.write(traceback.format_exc())
@@ -893,6 +936,8 @@ def run_gpu(opt):
                                         "(`latency` = one frame at a time); per-kernel roofline numbers come from an eager, event-instrumented pass")
         if not graphed:
             line["config"]["launch"] = "eager launches, one stream (no CUDA graph: --no-graph or the capture failed, see stderr)"
+        if dumped is not None:
+            write_outputs(dumped, opt.dump_outputs)
         sys.stdout.flush()
         os.write(real_stdout, (json.dumps(line) + "\n").encode())
     if world > 1:
@@ -1002,7 +1047,7 @@ def agent_sharded_leg(opt, rank, world, dev, peaks):
     wname = "c5" if n_agents == 8 else "c2"
     scenes = build_scenes(wname, 4, n_agents, seed0=500)              # the SAME scenes on every rank
     wl = GpuWorkload(wname, opt.precision, dev, n_agents=n_agents, scenes=scenes)
-    steps = max(opt.steps, 10)
+    steps = opt.steps
     with torch.no_grad():
         sf = parallel.AgentShardedFrame(wl.model, n_agents, rank, world, wl.cap, scenes[0]["pairwise"].shape, device=dev,
                                         comm=os.environ.get("HEAL_SHARD_COMM", "auto"))

@@ -181,6 +181,8 @@ def main():
     print("heter_model_baseline_att_small:", {k: tuple(v.shape) for k, v in bout.items() if torch.is_tensor(v)})
     make_convnext_golden()
     make_postprocess_golden()
+    make_point_filter_golden()
+    make_full_size_golden()
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)) // 1024, "KiB")
 
@@ -282,6 +284,90 @@ def make_postprocess_golden():
     multi["iou"] = {"cavs": [{"cls": cls, "reg": reg, "dir": dirp, "iou": iou, "T": T}], "boxes": boxes, "scores": scores}
     print("postprocess iou -> kept", boxes.shape[0])
     torch.save({"params": params, "anchors": anchors, "cases": cases, "multi": multi}, os.path.join(OUT, "postprocess.pt"))
+
+
+def point_filter_cloud():
+    """(20000, 4) cloud with plenty of points in and around the ego box and on the range / ego-box edges."""
+    rng = np.random.default_rng(5)
+    pts = rng.uniform(-120, 120, size=(20000, 4)).astype(np.float32)
+    pts[:, 2] = rng.uniform(-4, 2, size=20000)
+    pts[:2000, :2] = rng.uniform(-3, 3, size=(2000, 2))
+    pts[2000:2006] = [[-1.95, 0, 0, 1], [2.95, 1.1, 0, 1], [102.4, 0, 0, 1], [0, -102.4, 0, 1], [5, 5, -3, 1], [5, 5, 1, 1]]
+    return pts
+
+
+POINT_FILTER_LIMIT = [-102.4, -102.4, -3, 102.4, 102.4, 1]
+
+
+def make_point_filter_golden():
+    """UNMODIFIED reference pcd_utils mask_points_by_range / mask_ego_points / shuffle_points (pcd_utils.py:41-95) on
+    point_filter_cloud().  Their outputs are stored as bit-packed row masks: over the cloud for the two filters, over the cloud
+    shuffled with np.random.seed(3) for shuffle -> ego mask -> range mask.  To read the masks off the reference's outputs, the
+    cloud gets its row index as a fifth column, which the filters carry along untouched (they read columns 0-2 only)."""
+    from unittest.mock import MagicMock
+    ref_shim.install()
+    sys.modules.setdefault("pypcd", MagicMock(name="pypcd"))
+    from opencood.utils import pcd_utils as ref
+    pts = point_filter_cloud()
+    n, lim = pts.shape[0], POINT_FILTER_LIMIT
+    tagged = np.concatenate([pts, np.arange(n, dtype=np.float32)[:, None]], 1)
+    np.random.seed(3)
+    perm = np.random.permutation(n)
+
+    def mask(out5, out4, order):
+        rows = out5[:, 4].astype(np.int64)
+        assert np.array_equal(pts[rows], out4)
+        m = np.isin(order, rows)
+        assert np.array_equal(order[m], rows)                      # the filters keep the order of their input
+        return np.packbits(m)
+    by_range = mask(ref.mask_points_by_range(tagged, lim), ref.mask_points_by_range(pts, lim), np.arange(n))
+    ego = mask(ref.mask_ego_points(tagged), ref.mask_ego_points(pts), np.arange(n))
+    np.random.seed(3)
+    s5 = ref.shuffle_points(tagged)
+    np.random.seed(3)
+    s4 = ref.shuffle_points(pts)
+    assert np.array_equal(s5[:, 4].astype(np.int64), perm)
+    chain = mask(ref.mask_points_by_range(ref.mask_ego_points(s5), lim), ref.mask_points_by_range(ref.mask_ego_points(s4), lim), perm)
+    np.savez_compressed(os.path.join(OUT, "point_filters.npz"), limit=np.asarray(lim, np.float64),
+                        by_range=by_range, ego=ego, shuffle_seed3_ego_range=chain)
+
+
+FULL_SIZE_SAMPLES = 8192        # values stored per head: keeps the files small
+FULL_SIZE_STRIDE = 104729       # prime: on the 256x256 heads the sample visits every (channel, row) pair and every column
+
+
+def full_size_sample_index(numel):
+    """Flat positions of the stored sample of a head with `numel` elements."""
+    return (np.arange(FULL_SIZE_SAMPLES, dtype=np.int64) * FULL_SIZE_STRIDE) % numel
+
+
+def make_full_size_golden():
+    """UNMODIFIED reference PointPillar (configs[0]) and HeterPyramidCollab (configs[1]) at full size on CPU, on the clouds
+    tests/test_gpu_fullsize.py feeds the CUDA path.  Stored per head: its shape, max |ref| over the whole head (the tolerance
+    scale) and the values at full_size_sample_index()."""
+    from oracle import ref_runner
+    from workloads import configs as wcfg, synth
+    torch.set_num_threads(max(1, min(32, os.cpu_count() or 1)))
+
+    def heads(out):
+        rec = {}
+        for k in ("cls_preds", "reg_preds", "dir_preds"):
+            v = out[k].detach().float()
+            idx = torch.from_numpy(full_size_sample_index(v.numel()))
+            rec[k] = {"shape": tuple(v.shape), "max_abs": float(v.abs().max()), "value": v.reshape(-1)[idx].clone()}
+        return rec
+    # C2: tests/test_gpu_fullsize.py::_scene(5) (seed 321, 64 x 1024 rays per agent)
+    sc = synth.scene(321, n_agents=5, max_cav=5, rings=64, azimuth=1024)
+    model, _ = ref_runner.build_model("heter_pyramid_collab", wcfg.c2_args())
+    data, _ = ref_runner.c2_data({"clouds": sc["points"], "pairwise": sc["pairwise_t_matrix"]}, 5)
+    torch.save({"shapes": procedural.shapes_of(model), "heads": heads(ref_runner.forward(model, data))},
+               os.path.join(OUT, "full_size_c2.pt"))
+    # C1: one 20 x 1000-ray cloud
+    cloud = synth.lidar_cloud(np.random.default_rng(77), rings=20, azimuth=1000)
+    model, _ = ref_runner.build_model("point_pillar", wcfg.c1_args())
+    data, _ = ref_runner.c1_data(cloud)
+    torch.save({"shapes": procedural.shapes_of(model), "heads": heads(ref_runner.forward(model, data))},
+               os.path.join(OUT, "full_size_c1.pt"))
 
 
 if __name__ == "__main__":

@@ -1,8 +1,10 @@
 """Full-size parity: the BASELINE.json configs at their real shapes (range +-102.4 m -> 512x512 pillars / 2048x2048x40 voxels,
-256x256 fusion map, 64-line clouds, 704x256 images), CUDA path vs the UNMODIFIED reference modules on CPU (C1, C2: oracle/_ref
-through oracle.ref_runner) or the oracle port (C3 SECOND: no spconv-free reference; C4: the reference's LiftSplatShoot constructor
-hard-codes CUDA).  Tolerances are north_star's: 1e-3 (fp32-equivalent tc32) and 1e-2 (bf16), relative to max(1, max|ref|)."""
+256x256 fusion map, 64-line clouds, 704x256 images), CUDA path vs the UNMODIFIED reference modules on CPU (C1, C2: their
+heads stored under tests/golden by oracle/make_golden.py) or the oracle port (C3 SECOND: no spconv-free reference; C4: the
+reference's LiftSplatShoot constructor hard-codes CUDA).  Tolerances are north_star's: 1e-3 (fp32-equivalent tc32) and
+1e-2 (bf16), relative to max(1, max|ref|)."""
 import copy
+import os
 
 import numpy as np
 import pytest
@@ -39,16 +41,26 @@ def _scene(n_agents, rings=64, azimuth=1024, seed=321):
     return sc, torch.from_numpy(pts).cuda(), torch.from_numpy(offs).cuda()
 
 
+def _check_golden(out, heads, tol, tag):
+    """`_check` against a golden file of the reference's heads (oracle/make_golden.py::make_full_size_golden): the tolerance scale
+    is max|ref| over the whole head, the error is taken at the stored sample of its elements."""
+    from oracle.make_golden import full_size_sample_index
+    for k in HEADS:
+        h = heads[k]
+        g = out[k].float().cpu()
+        assert tuple(g.shape) == tuple(h["shape"]), (tag, k, g.shape, h["shape"])
+        err = (g.reshape(-1)[torch.from_numpy(full_size_sample_index(g.numel()))] - h["value"]).abs().max().item()
+        scale = max(h["max_abs"], 1.0)
+        print(f"{tag}/{k}: max|ref|={scale:.3f} max_abs_err={err:.3e} over {h['value'].numel()} samples (tol {tol * scale:.3e})")
+        assert err <= tol * scale, (tag, k, err, scale)
+
+
 @pytest.fixture(scope="module")
-def c2_reference():
-    """One full-size 5-agent frame through the unmodified reference HeterPyramidCollab on CPU (~10 s)."""
-    from oracle import ref_runner
-    assert ref_runner.available(), "oracle/_ref missing: python -m oracle.build_ref (build container)"
+def c2_reference(golden_dir):
+    """One full-size 5-agent frame through the unmodified reference HeterPyramidCollab on CPU, stored in full_size_c2.pt."""
+    g = torch.load(os.path.join(golden_dir, "full_size_c2.pt"), weights_only=False)
     sc, pts, offs = _scene(5)
-    model, sd = ref_runner.build_model("heter_pyramid_collab", wcfg.c2_args())
-    data, _ = ref_runner.c2_data({"clouds": sc["points"], "pairwise": sc["pairwise_t_matrix"]}, 5)
-    ref = ref_runner.forward(model, data)
-    return sc, pts, offs, sd, {k: ref[k] for k in HEADS}
+    return sc, pts, offs, procedural.make_state_dict(g["shapes"]), g["heads"]
 
 
 BF16_TOL = 2.5e-2      # see tests/test_gpu_models.py: bf16 storage noise through ~60 stored tensors; tc32 is the 1e-3 path
@@ -58,7 +70,7 @@ BF16_TOL = 2.5e-2      # see tests/test_gpu_models.py: bf16 storage noise throug
 def test_c2_full_size_vs_unmodified_reference(c2_reference, prec, tol):
     from heal_b200 import engine
     from heal_b200.models.heter_pyramid_collab import HeterPyramidCollab
-    sc, pts, offs, sd, ref = c2_reference
+    sc, pts, offs, sd, heads = c2_reference
     engine.set_precision(prec)
     m = HeterPyramidCollab(wcfg.c2_args()).eval()
     m.load_state_dict(sd, strict=True)
@@ -67,26 +79,25 @@ def test_c2_full_size_vs_unmodified_reference(c2_reference, prec, tol):
             "pairwise_t_matrix": torch.from_numpy(sc["pairwise_t_matrix"]).cuda()}
     with torch.no_grad():
         out = m(data)
-    _check(out, ref, tol, f"C2-full/{prec}")
+    _check_golden(out, heads, tol, f"C2-full/{prec}")
 
 
-def test_c1_full_size_vs_unmodified_reference():
-    """configs[0]: models/point_pillar.py, one 20k-ray cloud, range +-102.4 m (512x512 pillars)."""
-    from oracle import ref_runner
+def test_c1_full_size_vs_unmodified_reference(golden_dir):
+    """configs[0]: models/point_pillar.py, one 20k-ray cloud, range +-102.4 m (512x512 pillars); the reference's heads are
+    stored in full_size_c1.pt."""
     from heal_b200 import engine
     from heal_b200.models.point_pillar import PointPillar
     engine.set_precision("tc32")
+    g = torch.load(os.path.join(golden_dir, "full_size_c1.pt"), weights_only=False)
     cloud = synth.lidar_cloud(np.random.default_rng(77), rings=20, azimuth=1000)
-    rm, sd = ref_runner.build_model("point_pillar", wcfg.c1_args())
-    data, _ = ref_runner.c1_data(cloud)
-    ref = ref_runner.forward(rm, data)
+    sd = procedural.make_state_dict(g["shapes"])
     m = PointPillar(wcfg.c1_args()).eval()
     m.load_state_dict(sd, strict=True)
     m = m.cuda()
     offs = torch.tensor([0, cloud.shape[0]], dtype=torch.int32).cuda()
     with torch.no_grad():
         out = m({"processed_lidar": {"points": torch.from_numpy(cloud).cuda(), "agent_offsets": offs}})
-    _check(out, ref, 1e-3, "C1-full/tc32")
+    _check_golden(out, g["heads"], 1e-3, "C1-full/tc32")
 
 
 def test_c1_gpu_point_filters_equal_host_filters():

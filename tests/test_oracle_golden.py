@@ -3,7 +3,6 @@
 import os
 
 import numpy as np
-import pytest
 import torch
 
 from oracle import nets, procedural
@@ -92,27 +91,16 @@ def test_convnext_aligner_oracle_vs_reference_golden(golden_dir):
     assert (y - g["y"]).abs().max().item() <= 1e-5
 
 
-def test_point_filters_match_reference():
-    """oracle/pcd.py vs the unmodified reference's pcd_utils (mask_points_by_range / mask_ego_points / shuffle_points)."""
-    import sys
-    from unittest.mock import MagicMock
-    from oracle import pcd, ref_shim
-    if not ref_shim.available():
-        pytest.skip("reference tree not present")
-    ref_shim.install()
-    sys.modules.setdefault("pypcd", MagicMock(name="pypcd"))
-    from opencood.utils import pcd_utils as ref
-    rng = np.random.default_rng(5)
-    pts = rng.uniform(-120, 120, size=(20000, 4)).astype(np.float32)
-    pts[:, 2] = rng.uniform(-4, 2, size=20000)
-    pts[:2000, :2] = rng.uniform(-3, 3, size=(2000, 2))          # plenty of points in and around the ego box
-    pts[2000:2006] = [[-1.95, 0, 0, 1], [2.95, 1.1, 0, 1], [102.4, 0, 0, 1], [0, -102.4, 0, 1], [5, 5, -3, 1], [5, 5, 1, 1]]   # edges
-    lim = [-102.4, -102.4, -3, 102.4, 102.4, 1]
-    assert np.array_equal(pcd.mask_points_by_range(pts, lim), ref.mask_points_by_range(pts, lim))
-    assert np.array_equal(pcd.mask_ego_points(pts), ref.mask_ego_points(pts))
-    np.random.seed(3)
-    shuffled = ref.shuffle_points(pts)
-    np.random.seed(3)
-    perm = np.random.permutation(pts.shape[0])
-    expect = ref.mask_points_by_range(ref.mask_ego_points(shuffled), lim)
+def test_point_filters_match_reference(golden_dir):
+    """oracle/pcd.py vs the unmodified reference's pcd_utils (mask_points_by_range / mask_ego_points / shuffle_points), whose
+    outputs point_filters.npz stores as row masks (oracle/make_golden.py::make_point_filter_golden)."""
+    from oracle import make_golden, pcd
+    g = np.load(os.path.join(golden_dir, "point_filters.npz"))
+    pts, lim = make_golden.point_filter_cloud(), g["limit"].tolist()
+    n = pts.shape[0]
+    assert np.array_equal(pcd.mask_points_by_range(pts, lim), pts[np.unpackbits(g["by_range"], count=n).astype(bool)])
+    assert np.array_equal(pcd.mask_ego_points(pts), pts[np.unpackbits(g["ego"], count=n).astype(bool)])
+    np.random.seed(3)                                             # the reference's shuffle_points draws np.random.permutation
+    perm = np.random.permutation(n)
+    expect = pts[perm][np.unpackbits(g["shuffle_seed3_ego_range"], count=n).astype(bool)]
     assert np.array_equal(pcd.filter_cloud(pts, lim, perm), expect)
