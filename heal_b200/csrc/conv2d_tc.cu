@@ -556,11 +556,12 @@ k_conv2d_tc(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
 
 // HEAL_TC_* measurement hooks (profiles/tc_experiment.py), read once per process instead of six getenv calls per launch.
 struct TcEnv {
-    int dbg, pdl, halo, bo, tma_store, res_tma, ring, deep, l2promo;
+    int dbg, pdl, halo, bo, tma_store, res_tma, ring, tapn, deep, l2promo;
     TcEnv() {
         auto geti = [](const char* n, int dflt) { const char* e = getenv(n); return e ? atoi(e) : dflt; };
         dbg = geti("HEAL_TC_DBG", 0); pdl = geti("HEAL_TC_PDL", 1); halo = geti("HEAL_TC_HALO", 1); bo = geti("HEAL_TC_BO", 0);
-        tma_store = geti("HEAL_TC_TMA_STORE", 1); res_tma = geti("HEAL_TC_RES_TMA", 1); ring = geti("HEAL_TC_RING", 1); deep = geti("HEAL_TC_DEEP", 0); l2promo = geti("HEAL_TC_L2PROMO", 128);
+        tma_store = geti("HEAL_TC_TMA_STORE", 1); res_tma = geti("HEAL_TC_RES_TMA", 1); ring = geti("HEAL_TC_RING", 1); tapn = geti("HEAL_TC_TAPN", 1);
+        deep = geti("HEAL_TC_DEEP", 0); l2promo = geti("HEAL_TC_L2PROMO", 128);
     }
 };
 const TcEnv& tc_env() { static const TcEnv e; return e; }
@@ -756,13 +757,44 @@ extern "C" int heal_conv2d_tc(const void* in_split, size_t in_plane_stride, int 
     if (p.halo && p.bdiag) p.res_tma = 0;      // <64,4,1>: register prefetch
     cudaStream_t st = (cudaStream_t)stream_;
     const int kblocks = (blockdiag ? 1 : p.kc_blocks) * taps;
+    // grouped 3x3 on maps 64 or 128 pixels wide with split weights: the horizontal taps stacked along N (gconv3x3_tapn.cu), 24 MMAs
+    // per 128-pixel x 64-channel unit instead of 72.  It needs its own activation box (one row, one plane, no halo) and weight box
+    // (the 3 taps of a kernel row per sub-block); the output map above already has the unit's shape.
+    if (env.tapn && p.bdiag && p.tma_out && !res_split && !res_f32 && kh == 3 && kw == 3 && stride == 1 && pad == 1 &&
+        (Wo == 64 || Wo == 128) && relu != 2 && Cin == Cout && coutp == Cout && w_planes == 2) {
+        {
+            cuuint64_t dims[5] = {(cuuint64_t)Cin, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N, (cuuint64_t)planes};
+            cuuint64_t strides[4] = {(cuuint64_t)in_cstride * 2, (cuuint64_t)W * in_cstride * 2, (cuuint64_t)H * W * in_cstride * 2,
+                                     (cuuint64_t)in_plane_stride * 2};
+            if (planes == 1) strides[3] = strides[2] * N;
+            cuuint32_t box[5] = {(cuuint32_t)BLOCK_K, (cuuint32_t)W, 1u, 1u, 1u};
+            cuuint32_t es[5] = {1, 1, 1, 1, 1};
+            void* base = (void*)((const __nv_bfloat16*)in_split + in_coffset);
+            if (enc(&tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    CU_TENSOR_MAP_SWIZZLE_128B, act_promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) return HEAL_ERR_DRIVER;
+        }
+        {
+            // [plane][tap * C + co][16 ci]: the box {16 ci, 16 co, 3 taps, 2 planes, 4 sub-blocks} lands as [sub-block][plane][tap][co]
+            cuuint64_t d[5] = {16, 16, 9, 2, (cuuint64_t)Cout / 16};
+            cuuint64_t st_[4] = {32, (cuuint64_t)Cout * 32, (cuuint64_t)w_rows * 32, 512};
+            cuuint32_t b[5] = {16u, 16u, 3u, 2u, 4u};
+            cuuint32_t es[5] = {1, 1, 1, 1, 1};
+            if (enc(&tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, (void*)w_diag, d, st_, b, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                    CU_TENSOR_MAP_SWIZZLE_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+                return HEAL_ERR_DRIVER;
+        }
+        RingP rp;
+        rp.N = N; rp.H = Ho; rp.W = Wo; rp.C = Cout; rp.planes = planes; rp.wplanes = w_planes; rp.relu = relu; rp.bias = bias;
+        rp.segs = 1; rp.seg_rows = Ho; rp.pdl = env.pdl; rp.dbg = p.dbg;
+        return heal_gconv3x3_tapn_launch(tmA, tmB, tmO, rp, st);
+    }
     // grouped 3x3 on maps at least 128 pixels wide: the row-ring kernel (conv3x3_ring.cu) reads every input row and the weights
     // once per CTA instead of three times / once per tile; it shares the three tensor maps built above
     if (env.ring && p.halo && p.bdiag && p.tma_out && !res_split && !res_f32 && (Wo % 128) == 0 && relu != 2 && Cin == Cout &&
         coutp == Cout && !p.dbg) {
         RingP rp;
         rp.N = N; rp.H = Ho; rp.W = Wo; rp.C = Cout; rp.planes = planes; rp.wplanes = w_planes; rp.relu = relu; rp.bias = bias;
-        rp.segs = 1; rp.seg_rows = Ho; rp.pdl = env.pdl;
+        rp.segs = 1; rp.seg_rows = Ho; rp.pdl = env.pdl; rp.dbg = 0;
         return heal_conv3x3_ring_launch(tmA, tmB, tmO, rp, st);
     }
     if (relu == 2) {        // GELU: 1x1 / 3x3 convs with >= 128 output channels and no residual (ConvNeXt pwconv1: dim -> 4 dim)
